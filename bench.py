@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the reference's CPU path (oracle port) on the host cores
+    python bench.py --dump-outputs DIR ...    # also writes the last timed step's outputs (see dump_outputs)
 
 One step = one batch of `--batch` synthetic 512x512x3 tiles through 5 ResNet-9 generators ("flat-5":
 out_i = G_i(tile)), seg quantise + posneg mask.  Prints ONE JSON line (rank 0).
@@ -58,7 +59,12 @@ def parse():
     ap.add_argument("--no-extras", action="store_true", help="inference: skip the configs.{train,unet256,wsi} sub-records and the library baseline")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-roofline-events", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="inference: after the timed steps, write what the last one returned as DIR/<name>.npy (float32)")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.workload != "inference" or args.impl != "b200"):
+        ap.error("--dump-outputs applies to the b200 inference workload only")
+    return args
 
 
 def peaks():
@@ -67,6 +73,25 @@ def peaks():
         d = json.load(open(p))
         return d.get("bf16_tflops_sustained", 1431.0), d.get("hbm_gbs", 6572.0), "measured"
     return 1400.0, 6650.0, "fallback"
+
+
+DUMP_SAMPLE = 1 << 21          # elements kept per array: the seven outputs of a step stay under 64 MB as float32
+
+
+def dump_outputs(path, outs):
+    """Writes what TilePipeline.forward_device returned (four modalities, seg, seg uint8, posneg mask) as
+    <path>/<name>.npy in float32.  An array of more than DUMP_SAMPLE elements is reduced to DUMP_SAMPLE of its flattened
+    elements at indices drawn once from a fixed seed (sorted), so that two builds run with the same arguments can be
+    compared element for element."""
+    import numpy as np
+    mods, seg, seg_u8, mask = outs
+    arrays = {**{f"mod{i + 1}": m for i, m in enumerate(mods)}, "seg": seg, "seg_u8": seg_u8, "mask": mask}
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        if t.numel() > DUMP_SAMPLE:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.float().cpu().numpy())
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -243,12 +268,14 @@ def main():
     e0.record()
     t_host0 = time.perf_counter()
     for k in range(args.steps):
-        pipe.forward_device(xs[k % n_rot])
+        outs = pipe.forward_device(xs[k % n_rot])
     t_host = time.perf_counter() - t_host0       # host enqueue time (launch-bound if close to the device time)
     e1.record()
     barrier()
     launches = ops.LAUNCHES["count"] - l0
     t_ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:          # graph replays return static buffers: read them before `pipe` runs again
+        dump_outputs(args.dump_outputs, outs)
     # ---- roofline passes: the same step issued eagerly with CUDA events around every ResNet-block conv launch (events
     # cannot sit inside the replayed graph).  (a) in-region: the same stream layout as the headline, so the kernel is timed
     # while the other chains' kernels co-run; (b) isolated: ONE stream, nothing co-running ------------------------------

@@ -225,29 +225,49 @@ REAL_TILE = "/root/reference/Datasets/Sample_Dataset/test_cli/22_2.png"         
 REAL_ROI = ("/root/reference/Sample_Large_Tissues/ROI_7.png", (120, 200, 1120, 800))   # BASELINE config 3: crop box (l, t, r, b)
 
 
+def webp_lossless(img):
+    """The image as lossless WebP bytes: the same pixels as a PNG in about two thirds of the space."""
+    import io
+    from PIL import Image
+    buf = io.BytesIO()
+    img.save(buf, format="WEBP", lossless=True, quality=100, method=6)
+    data = buf.getvalue()
+    assert np.array_equal(np.asarray(Image.open(io.BytesIO(data)).convert("RGB")), np.asarray(img))
+    return np.frombuffer(data, dtype=np.uint8)
+
+
 def realtile_fixture():
     """BASELINE configs[0]: the reference's `deepliif test` body (infer_modalities, cli.py:833-919) on the REAL sample tile
     Datasets/Sample_Dataset/test_cli/22_2.png — PIL decode, transform, is_empty on real content, the nine generators, seg
-    aggregation, tensor2im, postprocess.  The PNG bytes travel inside the fixture (the GPU box has no /root/reference).
-    Stored at full resolution: Seg and Marker (the inputs of the mask / scoring); the other outputs 2x subsampled + sums."""
+    aggregation, tensor2im, postprocess.  The tile's pixels travel inside the fixture as lossless WebP.  Stored at full
+    resolution: the posneg mask of Seg, SegRefined, and SegOverlaid as its difference from the tile (mostly zero); Seg
+    and Marker 2x subsampled, the other outputs 4x; sums of every output."""
     import io
     from PIL import Image
     import_reference()
     import deepliif.models as RM
+    import deepliif.postprocessing as RP
     import deepliif.util as RU
     mdir = _e2e_model_dir()
-    png = open(REAL_TILE, "rb").read()
-    img = Image.open(io.BytesIO(png)).convert("RGB")
+    webp = webp_lossless(Image.open(REAL_TILE).convert("RGB"))
+    img = Image.open(io.BytesIO(webp.tobytes())).convert("RGB")
     torch.set_num_threads(os.cpu_count())
     images, scoring = RM.infer_modalities(img, 512, mdir, eager_mode=True, return_seg_intermediate=True)
-    arrs = {"png": np.frombuffer(png, dtype=np.uint8),
+    arrs = {"webp": webp,
             "names": np.frombuffer(json.dumps(sorted(images)).encode(), dtype=np.uint8),
             "scoring": np.frombuffer(json.dumps(scoring, sort_keys=True).encode(), dtype=np.uint8),
-            "variance": np.array(RU.image_variance_gray(img)), "is_empty": np.array(bool(RM.is_empty(img)))}
+            "variance": np.array(RU.image_variance_gray(img)), "is_empty": np.array(bool(RM.is_empty(img))),
+            "Seg__mask": RP.create_posneg_mask(np.asarray(images["Seg"]), 120)}
+    assert np.array_equal(arrs["Seg__mask"], pixel.create_posneg_mask(np.asarray(images["Seg"])))
     for k, im in images.items():
         a = np.asarray(im)
-        full = k in ("Seg", "mod4-Marker", "SegOverlaid", "SegRefined")
-        arrs[f"{k}__full" if full else f"{k}__sub2"] = a.copy() if full else a[::2, ::2].copy()
+        if k == "SegRefined":
+            arrs[f"{k}__full"] = a.copy()
+        elif k == "SegOverlaid":
+            arrs[f"{k}__minus_input"] = a - np.asarray(img)            # uint8, modulo 256
+        else:
+            st = 2 if k in ("Seg", "mod4-Marker") else 4
+            arrs[f"{k}__sub{st}"] = a[::st, ::st].copy()
         arrs[f"{k}__sum"] = checksum(a)
         arrs[f"{k}__shape"] = np.array(a.shape)
     print("real tile outputs:", sorted(images), scoring)
@@ -257,8 +277,8 @@ def realtile_fixture():
 def wsi_fixture():
     """BASELINE configs[2]: the reference's inference() (models/__init__.py:464-579: InferenceTiler, run_dask per tile,
     stitching) at tile_size=512, overlap_size=56 on a REAL 1000 x 600 region of Sample_Large_Tissues/ROI_7.png (6 tiles),
-    plus the InferenceTiler tile counts of all five ROIs at overlap 56 and 32.  Stored: the region as PNG bytes, Seg and
-    Marker 2x subsampled + sums, the other outputs 4x subsampled + sums."""
+    plus the InferenceTiler tile counts of all five ROIs at overlap 56 and 32.  Stored: the region as lossless WebP, Seg
+    and Marker 4x subsampled + sums, the other outputs 8x subsampled + sums."""
     import io
     from PIL import Image
     import_reference()
@@ -266,10 +286,8 @@ def wsi_fixture():
     import deepliif.util as RU
     mdir = _e2e_model_dir()
     path, box = REAL_ROI
-    region = Image.open(path).convert("RGB").crop(box)
-    buf = io.BytesIO(); region.save(buf, format="PNG", optimize=True)
-    png = buf.getvalue()
-    img = Image.open(io.BytesIO(png)).convert("RGB")
+    webp = webp_lossless(Image.open(path).convert("RGB").crop(box))
+    img = Image.open(io.BytesIO(webp.tobytes())).convert("RGB")
     torch.set_num_threads(os.cpu_count())
     opt = RM.get_opt(mdir)
     images = RM.inference(img, tile_size=512, overlap_size=56, model_path=mdir, eager_mode=True, opt=opt,
@@ -281,12 +299,12 @@ def wsi_fixture():
         counts[os.path.basename(f)] = {"size": list(im.size),
                                        "tiles_overlap56": sum(1 for _ in RU.InferenceTiler(im, 512, 56)),
                                        "tiles_overlap32": sum(1 for _ in RU.InferenceTiler(im, 512, 32))}
-    arrs = {"png": np.frombuffer(png, dtype=np.uint8), "names": np.frombuffer(json.dumps(sorted(images)).encode(), dtype=np.uint8),
+    arrs = {"webp": webp, "names": np.frombuffer(json.dumps(sorted(images)).encode(), dtype=np.uint8),
             "roi_tile_counts": np.frombuffer(json.dumps(counts, sort_keys=True).encode(), dtype=np.uint8),
             "n_tiles": np.array(sum(1 for _ in RU.InferenceTiler(img, 512, 56)))}
     for k, im in images.items():
         a = np.asarray(im)
-        st = 2 if k in ("Seg", "mod4-Marker") else 4
+        st = 4 if k in ("Seg", "mod4-Marker") else 8
         arrs[f"{k}__sub{st}"] = a[::st, ::st].copy()
         arrs[f"{k}__sum"] = checksum(a)
         arrs[f"{k}__shape"] = np.array(a.shape)
@@ -437,7 +455,9 @@ INIT_CASES = [("G", "resnet_9blocks", "batch", True), ("G", "unet_512", "batch",
 
 
 def init_signature(networks_module, case, seed=3):
-    """Per-tensor (sum, sum of |.|, first element) of a freshly initialised network under torch.manual_seed(seed)."""
+    """Per-tensor SHA-256 of the raw values of a freshly initialised network under torch.manual_seed(seed).  Exact, unlike
+    a floating-point sum, whose last bits depend on how many threads torch splits the reduction over."""
+    import hashlib
     kind, arch, norm, extra = case
     torch.manual_seed(seed)
     if kind == "G":
@@ -446,8 +466,7 @@ def init_signature(networks_module, case, seed=3):
         net = networks_module.define_D(6, 64, arch, extra, norm, "normal", 0.02, [])
     sd = net.state_dict()
     keys = list(sd)
-    sig = np.array([[float(v.double().sum()), float(v.double().abs().sum()), float(v.reshape(-1)[0])] if v.numel() else [0, 0, 0]
-                    for v in sd.values()], dtype=np.float64)
+    sig = [hashlib.sha256(v.detach().contiguous().numpy().tobytes()).hexdigest() for v in sd.values()]
     return keys, sig
 
 
@@ -458,7 +477,7 @@ def init_fixture():
     for i, case in enumerate(INIT_CASES):
         keys, sig = init_signature(N, case)
         arrs[f"c{i}_keys"] = np.frombuffer(json.dumps(keys).encode(), dtype=np.uint8)
-        arrs[f"c{i}_sig"] = sig
+        arrs[f"c{i}_sig"] = np.frombuffer(json.dumps(sig).encode(), dtype=np.uint8)
     save("init_weights", **arrs)
 
 
