@@ -377,6 +377,7 @@ extern "C" int dlb_conv_tc_fwd_stem(const float* x_nchw, int N, int C, int H, in
 extern "C" int dlb_conv_direct_fwd(const dlb_conv_desc* d, const float* x, int in_nchw, const float* in_scale,
                                    const float* in_shift, int in_act, const float* w_packed, const float* bias,
                                    float* y, int out_act, int out_nchw, dlb_stream_t stream) {
+  if (x == nullptr) return set_error("dlb_conv_direct_fwd: x is null");
   int OH, OW;
   if (out_shape(d, &OH, &OW) != 0) return DLB_ERR_INVALID;
   if (d->nsrc != 1) return set_error("dlb_conv_direct_fwd: single source only");

@@ -86,6 +86,74 @@ class Lazy:
                     border=border, border_mode=border_mode)
 
 
+@dataclass(frozen=True)
+class ResnetSwitches:
+    """The DLB_* kernel-path switches of ResnetEngine, read from the environment when an engine is built."""
+    fused: bool = True           # DLB_FUSED: fused-operand forward (norm + activation evaluated by the consuming conv)
+    fuse_residual: bool = True   # DLB_FUSE_RESIDUAL: the next block's first conv also evaluates the skip add
+    stem_stream: bool = True     # DLB_STEM_STREAM: row-streaming stem kernel (dlb_stem_conv_fwd)
+    head_stream: bool = True     # DLB_HEAD_STREAM: row-streaming head kernel (dlb_head_conv_fwd)
+    fuse_stem: bool = True       # DLB_FUSE_STEM: window operand built in shared memory (dlb_conv_tc_fwd_stem)
+    # measured: 0.99 ms fused (TMA-staged) vs 0.67 ms apply + TMA conv for up1
+    fuse_up: bool = False        # DLB_FUSE_UP: ConvTranspose convs read a fused operand
+    fuse_head: bool = True       # DLB_FUSE_HEAD: the non-streaming head reads a fused operand
+
+    @staticmethod
+    def from_env(fused=None, fuse_residual=None):
+        """fused / fuse_residual: explicit values override the environment."""
+        return ResnetSwitches(
+            fused=_env_flag("DLB_FUSED", True) if fused is None else bool(fused),
+            fuse_residual=_env_flag("DLB_FUSE_RESIDUAL", True) if fuse_residual is None else bool(fuse_residual),
+            stem_stream=_env_flag("DLB_STEM_STREAM", True), head_stream=_env_flag("DLB_HEAD_STREAM", True),
+            fuse_stem=_env_flag("DLB_FUSE_STEM", True), fuse_up=_env_flag("DLB_FUSE_UP", False),
+            fuse_head=_env_flag("DLB_FUSE_HEAD", True))
+
+
+@dataclass(frozen=True)
+class ResnetPlan:
+    """Which ResnetEngine code path runs for one input size."""
+    fused: bool   # True: _forward_fused; False: the layer-by-layer forward
+    stem: str     # "stream" (stem_conv) | "tc_stem" (conv_tc_stem) | "window" (stem_window_pack + conv_tc) | "direct"
+    head: str     # "stream" (head_conv) | "tc" (conv_tc[_fused] + head_finish) | "direct"
+
+
+def _resnet_kernels(stem_shape, head_shape, prec, backend, sw):
+    """Size-independent part of the plan: (stem_tc, stem_stream, head_tc, head_stream) for the stem / head weights
+    (PyTorch Conv2d shapes (Cout, Cin, R, S))."""
+    tc = backend == "tc"
+    co, ci, R, S = stem_shape
+    # stem on the tensor cores through the horizontal-window operand (K = 7 taps x 8 channel lanes = 64)
+    stem_tc = tc and ci <= 8 and S <= 8 and co % 32 == 0
+    # row-streaming stem kernel (dlb_stem_conv_fwd): C <= 4 -> 64, 7 x 7, split bf16
+    stem_stream = (stem_tc and sw.stem_stream and co == 64 and ci <= 4 and R == 7 and S == 7
+                   and prec.split and prec.fmt == FMT_BF16)
+    co, ci, R, S = head_shape
+    # head on the tensor cores with the horizontal taps moved into 32 virtual output channels (j = s*4 + co)
+    head_tc = tc and co <= 4 and S <= 8 and ci % 64 == 0
+    # row-streaming head kernel (dlb_head_conv_fwd): 64 -> co <= 3, 7 x 7, split bf16
+    head_stream = (head_tc and sw.head_stream and ci == 64 and R == 7 and S == 7 and co <= 3
+                   and prec.split and prec.fmt == FMT_BF16)
+    return stem_tc, stem_stream, head_tc, head_stream
+
+
+def resnet_plan(H, W, stem_shape, head_shape, precision="bf16x3", backend="tc", switches=None):
+    """The forward, stem and head ResnetEngine runs for an [N, C, H, W] input.  stem_shape / head_shape: shapes of the
+    generator's first and last Conv2d weights; switches: ResnetSwitches (default: read from the environment).  Needs no
+    weights and no device.  The per-layer choice between halo-strip and normalise-then-conv stays with the layer."""
+    prec = Precision.parse(precision) if isinstance(precision, str) else precision
+    sw = ResnetSwitches.from_env() if switches is None else switches
+    stem_tc, stem_stream, head_tc, head_stream = _resnet_kernels(stem_shape, head_shape, prec, backend, sw)
+    if not (backend == "tc" and sw.fused and stem_tc and head_tc and H % 4 == 0 and W % 4 == 0):
+        return ResnetPlan(False, "window" if stem_tc else "direct", "tc" if head_tc else "direct")
+    if stem_stream and H >= 8 and W >= 8 and (W >= 32 or H <= 256):   # (one statistics slice per row tile must fit the workspace)
+        stem = "stream"
+    elif sw.fuse_stem and stem_shape[1] <= 4 and H >= 16 and W >= 8 and stem_shape[3] == 7:
+        stem = "tc_stem"
+    else:
+        stem = "window"
+    return ResnetPlan(True, stem, "stream" if head_stream and H >= 8 and W >= 8 else "tc")
+
+
 def _tc_ok(cins, cout):
     return all(c % 64 == 0 for c in cins) and cout % 32 == 0
 
@@ -109,6 +177,7 @@ class ConvLayer:
         self.use_tc = backend == "tc" and _tc_ok(self.cins, self.cout)
         self.w_f32 = w          # kept for the data-gradient packing (training)
         d = ops.conv_desc(1, 8, 8, self.cins, self.cout, self.R, self.S, stride, pad, transposed, output_padding)
+        self.w_packed = None
         if self.use_tc:
             self.w_hi, self.w_lo = ops.pack_weights_tc(d, w, prec.fmt, prec.split)
         else:
@@ -166,6 +235,9 @@ class ConvLayer:
     def run_direct(self, x, N, H, W, *, pad_mode=PAD_ZERO, in_nchw=False, in_scale=None, in_shift=None,
                    in_act=ACT_NONE, out_act=ACT_NONE, out_nchw=False):
         d = self.desc(N, H, W, None, pad_mode)
+        if self.w_packed is None:       # a tensor-core layer that meets a shape its kernel does not take: packed once
+            assert len(self.cins) == 1, "direct kernel takes one source"
+            self.w_packed = ops.pack_weights_direct(d, self.w_f32)
         return ops.conv_direct(d, x, self.w_packed, self.bias, in_nchw, in_scale, in_shift, in_act, out_act, out_nchw)
 
 
@@ -233,13 +305,9 @@ class ResnetEngine(_EngineBase):
         super().__init__(norm, norm_mode, prec, backend, device)
         # fused operand load (default on the tensor-core backend): norm + activation (+ skip add) are evaluated by the
         # consuming convolution; fuse_residual also folds the ResnetBlock skip add into the next block's first conv.
-        self.fused = (backend == "tc") and (_env_flag("DLB_FUSED", True) if fused is None else bool(fused))
-        self.fuse_residual = _env_flag("DLB_FUSE_RESIDUAL", True) if fuse_residual is None else bool(fuse_residual)
         # per-stage switches (measured choices, see DESIGN.md): the trunk always gains; the stem / head / ConvTranspose stages
         # have little MMA work per converted strip and are converter-bound
-        self.fuse_stem = _env_flag("DLB_FUSE_STEM", True)
-        self.fuse_up = _env_flag("DLB_FUSE_UP", False)      # measured: 0.99 ms fused (TMA-staged) vs 0.67 ms apply + TMA conv for up1
-        self.fuse_head = _env_flag("DLB_FUSE_HEAD", True)
+        self.switches = ResnetSwitches.from_env(fused, fuse_residual)
         if padding_type not in ("zero", "reflect"):
             raise NotImplementedError("padding [%s] is not implemented" % padding_type)
         self.n_blocks, self.padding_type = n_blocks, padding_type
@@ -250,8 +318,11 @@ class ResnetEngine(_EngineBase):
         # stem: on the tensor cores through the horizontal-window operand (K = 7 taps x 8 channel lanes = 64),
         # else (validation backend / exotic channel counts) on the fp32 direct kernel.  head: direct kernel.
         w1 = g("model.1.weight")
-        self.stem_stream = False
-        self.stem_tc = backend == "tc" and w1.shape[1] <= 8 and w1.shape[3] <= 8 and w1.shape[0] % 32 == 0
+        idx_head = 4 + 3 * 2 + n_blocks + 3 * 2 + 1
+        wh, bh = g(f"model.{idx_head}.weight"), g(f"model.{idx_head}.bias")
+        self.stem_shape, self.head_shape = tuple(w1.shape), tuple(wh.shape)
+        self.stem_tc, self.stem_stream, self.head_tc, self.head_stream = _resnet_kernels(
+            self.stem_shape, self.head_shape, prec, backend, self.switches)
         if self.stem_tc:
             co, ci, R, S = w1.shape
             wk = torch.zeros((co, 64, R, 1), dtype=torch.float32, device=device)
@@ -259,9 +330,6 @@ class ResnetEngine(_EngineBase):
             wk.view(co, 8, 8, R)[:, :S, :ci, :] = w1.to(torch.float32).permute(0, 3, 1, 2)
             self.stem = ConvLayer(wk, g("model.1.bias"), pad=0, prec=prec, backend="tc", n_tile=n_tile)
             self.stem_S, self.stem_in_nc = S, ci
-            # row-streaming stem kernel (dlb_stem_conv_fwd): C <= 4 -> 64, 7 x 7, split bf16
-            self.stem_stream = (_env_flag("DLB_STEM_STREAM", True) and co == 64 and ci <= 4 and R == 7 and S == 7
-                                and prec.split and prec.fmt == FMT_BF16)
             self.stem_wpk = ops.stem_conv_pack(w1) if self.stem_stream else None
         else:
             self.stem = ConvLayer(w1, g("model.1.bias"), pad=3, backend="direct")
@@ -285,12 +353,8 @@ class ResnetEngine(_EngineBase):
             self.up.append(mk(f"model.{idx}", transposed=True, stride=2, pad=1, output_padding=1))
             self.up_norm.append(nrm(f"model.{idx + 1}"))
             idx += 3
-        idx += 1
         # head: on the tensor cores with the horizontal taps moved into 32 virtual output channels (j = s*4 + co),
         # followed by the shifted-sum finish; else the fp32 direct kernel.
-        wh, bh = g(f"model.{idx}.weight"), g(f"model.{idx}.bias")
-        self.head_tc = backend == "tc" and wh.shape[0] <= 4 and wh.shape[3] <= 8 and wh.shape[1] % 64 == 0
-        self.head_stream = False
         if self.head_tc:
             co, ci, R, S = wh.shape
             wv = torch.zeros((32, ci, R, 1), dtype=torch.float32, device=device)
@@ -299,9 +363,6 @@ class ResnetEngine(_EngineBase):
             self.head = ConvLayer(wv, None, pad=0, prec=prec, backend="tc", n_tile=32)
             self.head_bias = bh.detach().to(torch.float32).contiguous() if bh is not None else None
             self.head_S, self.head_co = S, co
-            # row-streaming head kernel (dlb_head_conv_fwd): 64 -> co <= 3, 7 x 7, split bf16
-            self.head_stream = (_env_flag("DLB_HEAD_STREAM", True) and ci == 64 and R == 7 and S == 7 and co <= 3
-                                and prec.split and prec.fmt == FMT_BF16)
             self.head_wpk = ops.head_conv_pack(wh) if self.head_stream else None
         else:
             self.head = ConvLayer(wh, bh, pad=3, backend="direct")
@@ -311,9 +372,10 @@ class ResnetEngine(_EngineBase):
         """x: fp32 NCHW [N,3,H,W] CUDA -> fp32 NCHW [N,3,H,W]."""
         x = x.contiguous()
         N, _, H, W = x.shape
+        plan = self.plan(H, W)
+        if plan.fused:
+            return self._forward_fused(x, plan, taps)
         tc = self.backend == "tc"
-        if tc and self.fused and self.stem_tc and self.head_tc and H % 4 == 0 and W % 4 == 0:
-            return self._forward_fused(x, taps)
         refl = self.pad_mode == PAD_REFLECT
         want = dict(want_f32=not tc, want_split=tc)
 
@@ -322,7 +384,7 @@ class ResnetEngine(_EngineBase):
                 taps[name] = a
 
         # stem: Pad3 + Conv7x7 (NCHW input read directly) -> norm -> ReLU
-        if self.stem_tc:
+        if plan.stem == "window":
             xh, xl = ops.stem_window_pack(x, 3, self.stem_S, self.pad_mode, self.prec.fmt, self.prec.split)
             y, ws = self.stem.run_tc([Act(None, xh, xl)], N, H + 6, W)
         else:
@@ -331,10 +393,15 @@ class ResnetEngine(_EngineBase):
         sc, sh = self._stats(y, self.stem_norm, ws)
         a = self._apply(y, sc, sh, ACT_RELU, **want)
         h, w = H, W
-        # two stride-2 down convs
+        # two stride-2 down convs (an odd extent gives ceil(h / 2): the extents are taken from each conv's output)
         for i in range(2):
-            y, ws = self._conv(self.down[i], a, N, h, w)
-            h, w = h // 2, w // 2
+            if tc and (h % 2 or w % 2):
+                # the tensor-core stride-2 conv takes even extents only: the fp32 direct kernel evaluates the previous
+                # layer's norm + ReLU while it loads that layer's raw output
+                y, ws = self.down[i].run_direct(y, N, h, w, in_scale=sc, in_shift=sh, in_act=ACT_RELU), None
+            else:
+                y, ws = self._conv(self.down[i], a, N, h, w)
+            h, w = y.shape[1], y.shape[2]
             sc, sh = self._stats(y, self.down_norm[i], ws)
             last = i == 1
             # the trunk keeps an fp32 residual stream next to the operand planes
@@ -363,18 +430,22 @@ class ResnetEngine(_EngineBase):
         # two ConvTranspose upsamplings
         for i in range(2):
             y, ws = self._conv(self.up[i], a, N, h, w)
-            h, w = h * 2, w * 2
+            h, w = y.shape[1], y.shape[2]
             sc, sh = self._stats(y, self.up_norm[i], ws)
             if i == 0:
                 a = self._apply(y, sc, sh, ACT_RELU, **want)
                 tap("up0", a)
         # head: (norm + ReLU fused into the load) Pad3 + Conv7x7 + bias + Tanh, NCHW out
-        if self.head_tc:
+        if plan.head == "tc":
             a = self._apply(y, sc, sh, ACT_RELU, pad=3, pad_mode=self.pad_mode)
             z, _ = self.head.run_tc([a], N, h + 6, w + 6, fuse_stats=False)
             return ops.head_finish(z, self.head_bias, w, self.head_S, self.head_co, ACT_TANH)
         return self.head.run_direct(y, N, h, w, pad_mode=self.pad_mode, in_scale=sc, in_shift=sh, in_act=ACT_RELU,
                                     out_act=ACT_TANH, out_nchw=True)
+
+    def plan(self, H, W):
+        """The forward / stem / head this engine runs for an [N, C, H, W] input (see resnet_plan)."""
+        return resnet_plan(H, W, self.stem_shape, self.head_shape, self.prec, self.backend, self.switches)
 
     def _consume(self, layer, lazy, N, H, W, *, pad=None, border=0, keep=False, fuse_stats=True, block=False, allow=(2,)):
         """Run `layer` on the lazy activation.  Strip-eligible layers evaluate it in-kernel (no HBM pass); the others
@@ -399,7 +470,7 @@ class ResnetEngine(_EngineBase):
         return y, ws, a.f32
 
     @torch.no_grad()
-    def _forward_fused(self, x, taps=None):
+    def _forward_fused(self, x, plan, taps=None):
         """The same network with (almost) no normalise/split pass between convolutions: a strip-eligible conv reads its
         producer's raw fp32 output and evaluates norm + ReLU (+ the block's skip add, + the reflect / zero border) while
         loading; with fuse_residual the skip add of block b is evaluated by the first conv of block b+1, which also
@@ -413,10 +484,10 @@ class ResnetEngine(_EngineBase):
             if taps is not None:
                 taps[name] = a
 
-        if self.stem_stream and H >= 8 and W >= 8 and (W >= 32 or H <= 256):   # (one statistics slice per row tile must fit the workspace)
+        if plan.stem == "stream":
             ws = ops.stats_workspace(N, H * W, self.stem.cout, x.device)
             y = ops.stem_conv(x, self.stem_wpk, self.stem.bias, self.stem.cout, self.pad_mode, stats_ws=ws)
-        elif self.fuse_stem and self.stem_in_nc <= 4 and H >= 16 and W >= 8 and self.stem_S == 7:
+        elif plan.stem == "tc_stem":
             ws = ops.stats_workspace(N, H * W, self.stem.cout, x.device)
             y = ops.conv_tc_stem(x, 3, self.stem_S, self.pad_mode, self.stem.cout, self.stem.w_hi, self.stem.w_lo, self.stem.bias,
                                  self.prec.fmt, self.prec.split, self.stem.n_tile, stats_ws=ws)
@@ -433,12 +504,15 @@ class ResnetEngine(_EngineBase):
             sc, sh = self._stats(y, self.down_norm[i], ws)
             cur = Lazy(y, sc, sh, ACT_RELU)
         for bi, (cv1, nm1, cv2, nm2) in enumerate(self.blocks):
-            if not self.fuse_residual and (cur.scale is not None or cur.residual is not None):
+            # the block input is also its skip operand: unless cur.x already holds it (no pending norm, activation or
+            # skip add), it is materialised in fp32
+            pending = cur.scale is not None or cur.residual is not None or cur.act != ACT_NONE
+            if not self.switches.fuse_residual and pending:
                 # separate skip-add pass: materialise r_b once, the first conv then loads it unchanged
                 r = self._apply(cur.x, cur.scale, cur.shift, cur.act, residual=cur.residual, want_f32=True, want_split=False).f32
                 cur = Lazy(r)
-            y, ws, r = self._consume(cv1, cur, N, h, w, pad=bpad, border=b, keep=cur.scale is not None or cur.residual is not None,
-                                     block=True)
+                pending = False
+            y, ws, r = self._consume(cv1, cur, N, h, w, pad=bpad, border=b, keep=pending, block=True)
             if r is None:
                 r = cur.x
             sc, sh = self._stats(y, nm1, ws)
@@ -447,14 +521,14 @@ class ResnetEngine(_EngineBase):
             cur = Lazy(y, sc, sh, ACT_NONE, residual=r)
             tap(f"block{bi}", cur)
         for i in range(2):
-            y, ws, _ = self._consume(self.up[i], cur, N, h, w, allow=(2, 4) if self.fuse_up else ())
+            y, ws, _ = self._consume(self.up[i], cur, N, h, w, allow=(2, 4) if self.switches.fuse_up else ())
             h, w = h * 2, w * 2
             sc, sh = self._stats(y, self.up_norm[i], ws)
             cur = Lazy(y, sc, sh, ACT_RELU)
-        if self.head_stream and cur.residual is None and h >= 8 and w >= 8:
+        if plan.head == "stream":
             return ops.head_conv(cur.x, cur.scale, cur.shift, cur.act, self.head_wpk, self.head_bias, self.head_co, self.pad_mode,
                                  ACT_TANH)
-        z, _, _ = self._consume(self.head, cur, N, h, w, border=3, fuse_stats=False, allow=(1, 2) if self.fuse_head else ())
+        z, _, _ = self._consume(self.head, cur, N, h, w, border=3, fuse_stats=False, allow=(1, 2) if self.switches.fuse_head else ())
         return ops.head_finish(z, self.head_bias, w, self.head_S, self.head_co, ACT_TANH)
 
     __call__ = forward

@@ -43,6 +43,13 @@ def _need_cuda(*ts):
             raise _lib.DeepliifB200Error("deepliif_b200 ops need contiguous CUDA tensors (no CPU path exists)")
 
 
+def _need_shape(what, t, shape):
+    """A tensor the kernel would index by the descriptor's extents must have exactly those extents: a mismatch is
+    refused here, before anything is launched."""
+    if t is not None and tuple(t.shape) != tuple(shape):
+        raise _lib.DeepliifB200Error(f"{what}: tensor of shape {tuple(t.shape)}, the descriptor needs {tuple(shape)}")
+
+
 def conv_desc(N, H, W, cins, Cout, R, S, stride=1, pad=0, transposed=False, output_padding=0, pad_mode=PAD_ZERO):
     cins = list(cins) if isinstance(cins, (list, tuple)) else [cins]
     arr = (C.c_int * 2)(*(cins + [0] * (2 - len(cins))))
@@ -98,6 +105,11 @@ def conv_tc(d, xs_hi, xs_lo, w_hi, w_lo, bias=None, fmt=FMT_BF16, split=True, n_
     xs_hi = list(xs_hi) if isinstance(xs_hi, (list, tuple)) else [xs_hi]
     xs_lo = (list(xs_lo) if isinstance(xs_lo, (list, tuple)) else [xs_lo]) if split else [None] * len(xs_hi)
     _need_cuda(*xs_hi, *xs_lo, w_hi, w_lo, bias)
+    if len(xs_hi) != d.nsrc:
+        raise _lib.DeepliifB200Error(f"conv_tc: {len(xs_hi)} sources, the descriptor has {d.nsrc}")
+    for s_, (xh, xl) in enumerate(zip(xs_hi, xs_lo)):
+        _need_shape(f"conv_tc source {s_}", xh, (d.N, d.H, d.W, d.Cin[s_]))
+        _need_shape(f"conv_tc source {s_} (lo)", xl, (d.N, d.H, d.W, d.Cin[s_]))
     oh, ow = conv_out_shape(d)
     if out is None:
         out = torch.empty((d.N, oh, ow, d.Cout), dtype=torch.float32, device=w_hi.device)
@@ -125,11 +137,17 @@ def conv_tc_fused(d, srcs, w_hi, w_lo, bias=None, fmt=FMT_BF16, split=True, n_ti
     out (fp32 NHWC or None: receives the evaluated operand), border, border_mode.  d.H / d.W include 2*border."""
     arr = (FusedSrc * 2)()
     keep = []
+    if len(srcs) != d.nsrc:
+        raise _lib.DeepliifB200Error(f"conv_tc_fused: {len(srcs)} sources, the descriptor has {d.nsrc}")
     for i, s_ in enumerate(srcs):
         x, sc, sh, res, o = s_["x"], s_.get("scale"), s_.get("shift"), s_.get("residual"), s_.get("out")
         _need_cuda(x, sc, sh, res, o)
         if x.dtype != torch.float32:
             raise _lib.DeepliifB200Error("conv_tc_fused: sources are fp32 NHWC tensors")
+        bd = int(s_.get("border", 0))
+        shape = (d.N, d.H - 2 * bd, d.W - 2 * bd, d.Cin[i])
+        for what, t in (("x", x), ("residual", res), ("out", o)):
+            _need_shape(f"conv_tc_fused source {i} {what}", t, shape)
         keep += [x, sc, sh, res, o]
         arr[i] = FusedSrc(x.data_ptr(), sc.data_ptr() if sc is not None else None, sh.data_ptr() if sh is not None else None,
                           int(s_.get("act", ACT_NONE)), res.data_ptr() if res is not None else None,
@@ -163,6 +181,8 @@ def conv_tc_stem(x_nchw, pad, S, pad_mode, cout, w_hi, w_lo, bias=None, fmt=FMT_
 def conv_direct(d, x, w_packed, bias=None, in_nchw=False, in_scale=None, in_shift=None, in_act=ACT_NONE,
                 out_act=ACT_NONE, out_nchw=False, out=None):
     _need_cuda(x, w_packed, bias, in_scale, in_shift)
+    cin = _cin_total(d)
+    _need_shape("conv_direct x", x, (d.N, cin, d.H, d.W) if in_nchw else (d.N, d.H, d.W, cin))
     oh, ow = conv_out_shape(d)
     if out is None:
         shape = (d.N, d.Cout, oh, ow) if out_nchw else (d.N, oh, ow, d.Cout)
@@ -327,6 +347,9 @@ def norm_apply(y, scale=None, shift=None, act=ACT_NONE, residual=None, want_f32=
     """out = act(y*scale+shift) (+ residual) -> (out_f32 | None, hi | None, lo | None)."""
     _need_cuda(y, scale, shift, residual)
     N, H, W, Cc = y.shape
+    _need_shape("norm_apply scale", scale, (N, Cc))
+    _need_shape("norm_apply shift", shift, (N, Cc))
+    _need_shape("norm_apply residual", residual, y.shape)
     f32 = torch.empty_like(y) if want_f32 else None
     hi = lo = None
     if want_split:

@@ -25,7 +25,7 @@ from . import ops
 
 
 class _Captured:
-    __slots__ = ("graph", "static_in", "outs", "launches")
+    __slots__ = ("graph", "static_in", "outs", "launches", "engines")
 
 
 class TilePipeline:
@@ -120,18 +120,30 @@ class TilePipeline:
         return self._stream_cache[key]
 
     # ---- CUDA-graph replay ----------------------------------------------------------------------------------------------
+    def _engines(self):
+        """The engine every network runs with now.  net.engine() rebuilds it when the network's weights or precision
+        changed, so a replay can tell whether its graph still matches the networks.  None for a plain callable."""
+        return [n.engine() if hasattr(n, "engine") else None for n in self.gens + (self.segs or []) if n is not None]
+
     def _graphed(self, kind, shape, dtype, dev, body):
         """Captured graph of `body(static_in)` for this input shape, or None the first time the shape is seen (the
-        caller then runs eagerly, which doubles as the warm-up that fills the workspace caches)."""
+        caller then runs eagerly, which doubles as the warm-up that fills the workspace caches).  A graph bakes in the
+        engines' weight buffers: once any network has rebuilt its engine, every graph is dropped and the shape starts
+        over (eager, then captured again)."""
         key = (kind, tuple(shape), dtype, str(dev), self._keep_parts is not None)
         cap = self._graphs.get(key)
         if cap is not None:
-            return cap
+            if all(a is b for a, b in zip(self._engines(), cap.engines)):
+                return cap
+            torch.cuda.synchronize()      # a replay still in flight reads the graph pool and the old weights
+            self._graphs.clear()
+            self._seen.clear()
         if key not in self._seen:
             self._seen.add(key)
             return None
         cap = _Captured()
         cap.static_in = torch.zeros(tuple(shape), dtype=dtype, device=dev)
+        cap.engines = self._engines()
         torch.cuda.synchronize()
         l0 = ops.LAUNCHES["count"]
         cap.graph = torch.cuda.CUDAGraph()
